@@ -15,6 +15,11 @@ image) on the host cores for the same config and prints the same JSON line with 
 
 Launch: python bench.py --gpus N --steps K --warmup W   (N > 1 under torch.distributed.run, one rank per GPU;
 scenes are sharded by rank -- weak scaling, per-GPU work fixed -- and the assigned track ids are gathered with NCCL).
+
+`--dump-outputs DIR` writes what the timed path returned for the last timed frame as DIR/<name>.npy (rank 0's shard):
+ids, epochs, lengths, voting_types of the device-pointer path and predicted_boxes, observed_boxes of the host-pointer
+path (with --impl reference: the oracle's ids, epochs, lengths, voting_types).  The frames are seeded, so two builds run
+with the same arguments can be compared array for array.
 """
 from __future__ import annotations
 
@@ -49,7 +54,35 @@ def parse():
                     help="override the visual metric's threshold: a float, or 'max' = the reference's default Euclidean(f32::MAX)")
     ap.add_argument("--feat-noise", type=float, default=None, help="override the workload's feature noise (sensitivity sweeps)")
     ap.add_argument("--no-scatter", action="store_true", help="N > 1: skip the ingest-rank scatter arm (sb200_shard_*)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step as DIR/<name>.npy (float32 / float64)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
+
+
+DUMP_LIMIT_BYTES = 64 * 10**6
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes the per-detection arrays of one frame as out_dir/<name>.npy: float64 where float32 could not hold every
+    value (ids, epochs, lengths), float32 otherwise.  When they would exceed DUMP_LIMIT_BYTES, a fixed, seeded sample of
+    the detections is written instead -- the same rows of every array, their indices in rows.npy."""
+    def as_float(a):
+        a = np.asarray(a)
+        return a.astype(np.float64 if a.dtype.kind in "iu" and a.dtype.itemsize >= 4 else np.float32)
+
+    arrays = {k: as_float(a) for k, a in arrays.items()}
+    n = len(next(iter(arrays.values())))
+    row_bytes = sum(a[:1].nbytes for a in arrays.values())
+    if n * row_bytes > DUMP_LIMIT_BYTES:
+        rows = np.sort(np.random.default_rng(0).choice(n, (DUMP_LIMIT_BYTES - 4096) // (row_bytes + 8), replace=False))
+        arrays = {k: a[rows] for k, a in arrays.items()}
+        arrays["rows"] = rows.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{k}.npy"), a)
 
 
 def config_dict(name, cfg, extra=None):
@@ -237,13 +270,14 @@ def option_overrides(args):
 
 
 def cpu_port_run(name, frames, warm, steps, threads, over=None):
-    """Times the oracle tracker (reference algorithm, reference execution order, `threads` host threads)."""
+    """Times the oracle tracker (reference algorithm, reference execution order, `threads` host threads).  Returns the
+    pair-associations and seconds of the timed frames and the result of the last frame."""
     import oracle as orc
     from similari_b200.workload import tracker_options_for
 
     opts = tracker_options_for(name, orc.make_options, **(over or {}))
     t = orc.Tracker(opts, threads=threads)
-    units, secs = 0, 0.0
+    units, secs, last = 0, 0.0, None
 
     def live_tracks(scene):
         # N of the metric = stored tracks that can still match (the reference keeps expired tracks in its store until
@@ -256,12 +290,12 @@ def cpu_port_run(name, frames, warm, steps, threads, over=None):
         m = np.diff(f["det_offsets"]).astype(np.int64)
         n_before = np.array([live_tracks(int(s)) for s in f["scene_ids"]], dtype=np.int64) if i >= warm else None
         t0 = time.perf_counter()
-        t.predict_batch(f["scene_ids"], f["det_offsets"], f["boxes"], features=f["features"], want_boxes=False)
+        last = t.predict_batch(f["scene_ids"], f["det_offsets"], f["boxes"], features=f["features"], want_boxes=False)
         dt = time.perf_counter() - t0
         if i >= warm:
             units += int((m * n_before).sum())
             secs += dt
-    return units, secs
+    return units, secs, last
 
 
 def run_reference(args):
@@ -280,9 +314,11 @@ def run_reference(args):
     full = CONFIGS[args.config].n_scenes
     sample_scenes = min(args.cpu_sample_scenes or full, full)
     warm = max(3, args.warmup)
-    steps = max(1, args.steps)
+    steps = args.steps
     cfg, frames = make_frames(args.config, warm + steps, 0, sample_scenes, feat_noise=args.feat_noise)
-    units, secs = cpu_port_run(args.config, frames, warm, steps, cores, option_overrides(args))
+    units, secs, last = cpu_port_run(args.config, frames, warm, steps, cores, option_overrides(args))
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {k: last[k] for k in ("ids", "epochs", "lengths", "voting_types")})
     value = units / secs
     line = {
         "impl": "reference", "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": args.gpus, "steps": steps,
@@ -542,7 +578,9 @@ def main():
     ev1.synchronize()
     sampler.mark_end()
     e2e_total_ms = float(ev0.elapsed_time(ev1))
-    ids_e2e_last = out_ring[(W + K - 1) % RING]["ids"][: len(frames[W + K - 1]["boxes"])].copy()
+    n_last = len(frames[W + K - 1]["boxes"])
+    e2e_last = {k: v[:n_last].copy() for k, v in out_ring[(W + K - 1) % RING].items()}
+    ids_e2e_last = e2e_last["ids"]
     t_e2e.close()
 
     # ---------------------------------------------------------------- value: inputs resident in HBM
@@ -619,8 +657,14 @@ def main():
     clocks = sampler.stop() if sampler else None
     launches = eng.launch_count() - l0
     c1 = t_dev.work_counters()
-    ids_dev_last = d_ids[(W + K - 1) & 1][: len(frames[W + K - 1]["boxes"])].cpu().numpy().astype(np.uint64)
+    b_last = (W + K - 1) & 1
+    ids_dev_last = d_ids[b_last][:n_last].cpu().numpy().astype(np.uint64)
     assert np.array_equal(ids_dev_last, ids_e2e_last), "device-pointer and host-pointer paths disagree"
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {
+            "ids": ids_dev_last, "epochs": d_ep[b_last][:n_last].cpu().numpy(),
+            "lengths": d_len[b_last][:n_last].cpu().numpy(), "voting_types": d_vt[b_last][:n_last].cpu().numpy(),
+            "predicted_boxes": e2e_last["predicted"], "observed_boxes": e2e_last["observed"]})
     if gather is not None:   # every rank holds every shard's ids of the last step
         gl = gather["buf"][(W + K - 1) & 1].view(world, max_total)[rank][: len(ids_dev_last)].cpu().numpy().astype(np.uint64)
         assert np.array_equal(gl, ids_dev_last), "gathered ids differ from the local shard"
@@ -747,7 +791,7 @@ def main():
             cores = usable_cores()
             sample = args.cpu_sample_scenes or min(cfg.n_scenes, max(cores, 64))
             ccfg, cframes = make_frames(name, 6, 0, sample, feat_noise=args.feat_noise)
-            cu, cs = cpu_port_run(name, cframes, 4, 2, cores, over)
+            cu, cs, _ = cpu_port_run(name, cframes, 4, 2, cores, over)
             line["cpu_baseline"] = {"value": cu / cs, "unit": UNIT, "cores": cores, "kind": "port",
                                     "sample": f"{sample} of {cfg.n_scenes} scenes x 2 timed frames after 4 warm-up frames, "
                                               f"{cores} threads (scene-parallel), {cs:.1f} s"}

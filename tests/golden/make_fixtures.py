@@ -1,5 +1,7 @@
-"""Builds the committed input fixtures from the reference's regression data (run once in the build container, where
-/root/reference exists; the GPU box only sees the .npz files).
+"""Builds the committed input fixtures from the reference's regression data.  The tests read only the .npz files;
+this script is run by hand against a checkout of insight-platform/Similari:
+
+  python tests/golden/make_fixtures.py <path to the Similari checkout>
 
   python/bugfixes/bug_vs_1/in/**/*.json  -> bug_vs_1.npz   (real 512-d re-id features, VisualSort; the reference
                                                              script asserts "a track id appears once per frame")
@@ -12,10 +14,11 @@ Only DATA is extracted (numbers), no reference code.  Boxes are stored as float3
 import ast
 import json
 import pathlib
+import sys
 
 import numpy as np
 
-REF = pathlib.Path("/root/reference/python/bugfixes")
+REF = None   # <checkout>/python/bugfixes, set from the command line
 OUT = pathlib.Path(__file__).parent
 
 
@@ -48,6 +51,9 @@ def github_84():
 
 
 if __name__ == "__main__":
+    if len(sys.argv) != 2:
+        raise SystemExit(__doc__)
+    REF = pathlib.Path(sys.argv[1]) / "python" / "bugfixes"
     bug_vs_1()
     github_84()
     for f in ("bug_vs_1.npz", "github_84.npz"):
